@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the FILM hot path: interpolated frames/sec (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -26,6 +26,10 @@ own frame pairs (frame pairs shard embarrassingly; no data-path collective) -> w
             the TF2 reference itself cannot run here -- no TensorFlow in the image). Every step is
             ONE REAL 1080p call of the oracle; the number of steps is capped by a wall budget and
             the line reports the steps actually timed.
+`--dump-outputs DIR`: after the timed steps, the mid-frame the timed path returned in its last step (rank 0's frame
+            pair) is written as DIR/mid_frame.npy, float32 (1, H, W, 3). Inputs and weights are seeded, so two builds
+            run with the same arguments can be compared value for value. A frame over DUMP_LIMIT_BYTES is replaced by
+            a seeded sample of its rows, DIR/mid_frame_sample.npy.
 """
 from __future__ import annotations
 
@@ -57,6 +61,25 @@ def load_peaks():
                 "source": "measured (MEASURED_PEAKS.json)"}
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0,
             "source": "fallback (B200_PROFILING.md)"}
+
+
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(outdir: str, frame: np.ndarray) -> str:
+    """Writes `frame` (B, H, W, 3) as <outdir>/mid_frame.npy in float32; over DUMP_LIMIT_BYTES, a sample of its rows
+    (drawn without replacement from default_rng(0), kept in order) as <outdir>/mid_frame_sample.npy instead."""
+    os.makedirs(outdir, exist_ok=True)
+    frame = np.ascontiguousarray(frame, dtype=np.float32)
+    name = "mid_frame"
+    if frame.nbytes > DUMP_LIMIT_BYTES - 4096:                     # 4 KB of room for the .npy header
+        row_bytes = frame.nbytes // frame.shape[1]
+        rows = np.sort(np.random.default_rng(0).choice(frame.shape[1], (DUMP_LIMIT_BYTES - 4096) // row_bytes,
+                                                       replace=False))
+        name, frame = "mid_frame_sample", np.ascontiguousarray(frame[:, rows])
+    path = os.path.join(outdir, name + ".npy")
+    np.save(path, frame)
+    return path
 
 
 class ClockSampler:
@@ -181,7 +204,7 @@ class CpuOracle1080p:
 
     def step(self) -> float:
         t = time.perf_counter()
-        self.orc.interpolate(self.x0, self.x1, self.dt)
+        self.out = self.orc.interpolate(self.x0, self.x1, self.dt)
         return time.perf_counter() - t
 
 
@@ -204,6 +227,8 @@ def run_reference(args):
         if secs and (time.perf_counter() - t_start) + 1.1 * float(np.mean(secs)) > REF_WALL_BUDGET_S:
             break
         secs.append(orc.step())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, orc.out)
     sec = float(np.mean(secs))
     v = 1.0 / sec
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "frames/s", "n_gpus": args.gpus,
@@ -357,7 +382,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-workloads", action="store_true", help="skip the 4K / 8K / 720p-recursive workloads")
     ap.add_argument("--op-table", default=None, help="write the per-kernel timing table (csv) here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the mid-frame of the last timed step as DIR/mid_frame.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -375,7 +404,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     W = max(args.warmup, 3)
-    K = max(args.steps, 1)
+    K = args.steps
     h, w = args.height, args.width
 
     eng = Interpolator("synthetic", align=64, device=local_rank)
@@ -418,6 +447,8 @@ def main():
     ms_total = float(t_ms.item())
     value = world * K / (ms_total / 1e3)
     prof = eng.profile()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dout.cpu().numpy())
 
     # ---- end to end through the reference-facing API (host buffers) -----------------
     hx0 = torch.from_numpy(x0).pin_memory().numpy()

@@ -174,10 +174,14 @@ def from_named_arrays(arrays: Mapping[str, np.ndarray], partial: bool = False) -
 
 
 def ensure_synthetic_file(path: str | None = None, seed: int = 1234) -> str:
-    """Write the synthetic weight file once (cache dir under the system temp dir) and return its path."""
+    """Write the synthetic weight file once (cache dir under the system temp dir) and return its path.
+
+    The default cache dir is per user: on a shared host the temp dir is shared, and a cache dir another user
+    created there is not writable."""
     if path is None:
         import tempfile
-        root = os.environ.get("FILM_B200_CACHE", os.path.join(tempfile.gettempdir(), "film_b200_cache"))
+        root = os.environ.get("FILM_B200_CACHE",
+                              os.path.join(tempfile.gettempdir(), f"film_b200_cache-{os.getuid()}"))
         os.makedirs(root, exist_ok=True)
         path = os.path.join(root, f"synthetic_seed{seed}.filmw")
     if not os.path.exists(path):

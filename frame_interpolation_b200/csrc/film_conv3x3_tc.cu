@@ -496,8 +496,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_conv3x3_tc(const ConvProblem* _
               const float a = f[j] + __shfl_xor_sync(0xffffffffu, f[j], 1);
               pf[j] = (a + __shfl_xor_sync(0xffffffffu, a, 8)) * 0.25f;
             }
-            // lanes with even tile row and even tile column own the pooled pixel (H, W are even)
-            if (valid && !(lane & 1) && !(lane & 8)) {
+            // lanes with even tile row and even tile column own the pooled pixel; VALID pooling floors, so on an
+            // odd-sized level the last row / column has no pooled pixel (its 2x2 window would leave the grid)
+            if (!(lane & 1) && !(lane & 8) && (py >> 1) < (out_H >> 1) && (px >> 1) < (out_W >> 1)) {
               const int64_t ppix = ((int64_t)b * (out_H >> 1) + (py >> 1)) * (out_W >> 1) + (px >> 1);
               pack_store16(pf, pool_hi + ppix * pool_C + n0 + cc * 16, pool_lo + ppix * pool_C + n0 + cc * 16);
             }

@@ -620,7 +620,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
               const float a = f[j] + __shfl_xor_sync(0xffffffffu, f[j], 1);
               pf[j] = (a + __shfl_xor_sync(0xffffffffu, a, 8)) * 0.25f;
             }
-            if (valid && !(lane & 1) && !(lane & 8)) {
+            // even-row, even-column lanes own the pooled pixel; VALID pooling floors (odd sizes drop the last row / column)
+            if (!(lane & 1) && !(lane & 8) && (py >> 1) < (out_H >> 1) && (px >> 1) < (out_W >> 1)) {
               const int64_t ppix = ((int64_t)b * (out_H >> 1) + (py >> 1)) * (out_W >> 1) + (px >> 1);
               pack_store16(pf, pool_hi + ppix * pool_C + n0 + cc * 16, pool_lo + ppix * pool_C + n0 + cc * 16);
             }

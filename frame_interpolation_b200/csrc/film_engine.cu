@@ -273,6 +273,14 @@ static std::vector<TapSpec> taps_up2x2(int py, int px) {
     }
   return t;
 }
+// the same 2x2 SAME conv on the fine grid (tap (ky,kx) reads offset (ky,kx); the bottom/right pad is the zero
+// fill of out-of-bounds reads): the decoder's general path, used where the fine level is not twice the coarse one
+static std::vector<TapSpec> taps_2x2() {
+  std::vector<TapSpec> t;
+  for (int ky = 0; ky < 2; ++ky)
+    for (int kx = 0; kx < 2; ++kx) t.push_back({ky, kx, {{ky, kx}}});
+  return t;
+}
 static std::vector<int> iota_map(int start, int n, int padded) {
   std::vector<int> m(padded, -1);
   for (int i = 0; i < n; ++i) m[i] = start + i;
@@ -303,6 +311,7 @@ struct Model {
   PackedConv flow_c3[4];                         // predictor p, 1x1 conv_3 (tensor-core, fused head)
   float *flow_w3[4], *flow_b3[4], *flow_w4[4], *flow_b4[4];
   PackedConv fus_up[4][4];                       // level i, parity class py*2+px
+  PackedConv fus_up_full[4];                     // level i, plain 2x2 conv on the fine grid (general path)
   PackedConv fus_c1[4], fus_c2[4];
   float *rgb_w = nullptr, *rgb_b = nullptr;
 
@@ -372,6 +381,7 @@ struct Model {
       for (int py = 0; py < 2; ++py)
         for (int px = 0; px < 2; ++px)
           fus_up[i][py * 2 + px] = pack_conv(k0, b0, up_src, taps_up2x2(py, px), allocs);
+      fus_up_full[i] = pack_conv(k0, b0, up_src, taps_2x2(), allocs);
       const int a_c = 2 * (3 + C) + 4;
       fus_c1[i] = pack_conv(get_tensor(w, pre + "1/kernel", {3, 3, a_c + nf, nf}),
                             get_tensor(w, pre + "1/bias", {nf}),
@@ -743,9 +753,31 @@ static size_t add_conv(Plan& P, const std::string& tag, double ref_macs_per_px, 
   return idx;
 }
 
+// eval/interpolator.py:30-63: network size (H, W) of an (h, w) frame and the offset of the frame inside it
+static void padded_size(int h, int w, int align, int& H, int& W, int& off_y, int& off_x) {
+  int ph = 0, pw = 0;
+  if (align > 0) {
+    ph = (h % align) ? align - h % align : 0;
+    pw = (w % align) ? align - w % align : 0;
+  }
+  H = h + ph;
+  W = w + pw;
+  off_y = ph / 2;
+  off_x = pw / 2;
+}
+
+// The reference graph accepts any size (VALID pooling floors, flows and the decoder resize to each level's size), and so
+// does this engine when the handle option "any_size" is on.  Without it a padded size that is not a multiple of 64 (what
+// the CLI default --align 64, eval/interpolator_cli.py:103, always gives) is refused.
+static void check_supported_size(int H, int W, bool any_size) {
+  if (!any_size && (H % 64 || W % 64))
+    throw Error{FILM_ERR_UNSUPPORTED,
+                "padded frame size must be a multiple of 64 (2^(pyramid_levels-1)) in this engine; use align=64"};
+}
+
 static std::unique_ptr<Plan> build_plan(const Model& M, int h, int w, int align, int conv_impl, bool keep_debug,
                                         int conv3x3_v2, int num_sms, int conv3x3_2cta, int conv3x3_halo,
-                                        uint32_t onepass_mask, bool use_lanes, int fe_conv0_tc) {
+                                        uint32_t onepass_mask, bool use_lanes, int fe_conv0_tc, bool any_size) {
   std::unique_ptr<Plan> pl(new Plan);
   Plan& P = *pl;
   P.fe_conv0_tc = fe_conv0_tc & 1;
@@ -763,21 +795,8 @@ static std::unique_ptr<Plan> build_plan(const Model& M, int h, int w, int align,
   P.conv3x3_2cta = conv3x3_2cta;
   P.conv3x3_halo = conv3x3_halo;
   P.num_sms = num_sms;
-  // eval/interpolator.py:30-63
-  int ph = 0, pw = 0;
-  if (align > 0) {
-    ph = (h % align) ? align - h % align : 0;
-    pw = (w % align) ? align - w % align : 0;
-  }
-  P.H = h + ph;
-  P.W = w + pw;
-  P.off_y = ph / 2;
-  P.off_x = pw / 2;
-  // The reference graph accepts any size (VALID pooling floors, flows and fusion resize to the level size);
-  // this engine implements the 64-aligned case only -- the CLI default (--align 64, eval/interpolator_cli.py:103).
-  if (P.H % 64 || P.W % 64)
-    throw Error{FILM_ERR_UNSUPPORTED,
-                "padded frame size must be a multiple of 64 (2^(pyramid_levels-1)) in this engine; use align=64"};
+  padded_size(h, w, align, P.H, P.W, P.off_y, P.off_x);
+  check_supported_size(P.H, P.W, any_size);
   int Hs[kLevels], Ws[kLevels];
   for (int l = 0; l < kLevels; ++l) {
     Hs[l] = P.H >> l;
@@ -1062,7 +1081,27 @@ static std::unique_ptr<Plan> build_plan(const Model& M, int h, int w, int align,
       up_src = {{batch_view(wf[i + 1], 0), 0}, {batch_view(wf[i + 1], 1), 0}, {side[i + 1], 0}};
     else
       up_src = {{net, 0}};
-    if (P.conv_impl == 0) {
+    if (hh != 2 * Hs[i + 1] || ww != 2 * Ws[i + 1]) {
+      // general path (a level of odd size below it: the fine grid is not twice the coarse one): every source is resized
+      // by nearest neighbour onto the fine grid, then the plain 2x2 SAME conv runs there (both conv_impl values)
+      const bool hi_only = P.conv_impl == 0 && P.plane_skip && ((P.onepass_mask >> (ST_FUS + 3 * i)) & 1u);
+      std::vector<SplitBuf*> resized;
+      for (size_t s = 0; s < up_src.size(); ++s) {
+        const SplitBuf* src = up_src[s].buf;
+        SplitBuf* dst = P.split(src->B, hh, ww, src->C);
+        const double rbytes = (double)src->B * src->C * 2.0 * (hi_only ? 1.0 : 2.0) * ((double)hh * ww + (double)src->H * src->W);
+        P.add_op(2, "fusion_resize" + std::to_string(s) + "@L" + std::to_string(i), [=](cudaStream_t st) {
+          return launch_resize_nearest(src->hi, src->lo, src->B, src->H, src->W, src->C, dst->hi, dst->lo, hh, ww, hi_only, st);
+        }, 0, rbytes);
+        P.debug["fusion_resized" + std::to_string(s) + "/" + std::to_string(i)] =
+            DebugTensor{true, dst->hi, dst->lo, (int64_t)hh * ww, dst->C, 0, dst->C};
+        up_src[s].buf = dst;
+        resized.push_back(dst);
+      }
+      add_conv(P, "fusion_up2x2@L" + std::to_string(i), 4.0 * M.fus_up_full[i].cin_ref * nf, M.fus_up_full[i], up_src, 0, up,
+               0, ST_FUS + 3 * i, ST_FUS + 3 * i + 1);
+      for (SplitBuf* r : resized) P.release(r);
+    } else if (P.conv_impl == 0) {
       // the four parity classes share the grid: ONE launch, grid.z = class
       size_t first = 0;
       for (int py = 0; py < 2; ++py)
@@ -1213,6 +1252,8 @@ struct film_handle {
                           // time in the same-box A/B of profiles/r2d_variants_ab.md)
   int plane_skip = 1, mma_straight = 1, arena_reuse = 1;   // round-2 optimisations, individually switchable (A/B, bisecting)
   int fuse_flow_head = 1;
+  int any_size = 0;     // 1 = padded frame sizes that are not multiples of 64 are computed (the reference graph's general
+                        // case); 0 (default) = they are refused with FILM_ERR_UNSUPPORTED.  Never changes a 64-aligned plan.
   uint8_t* u8_stage = nullptr;  // film_interpolate_u8: [x0][x1][out] on the device
   size_t u8_bytes = 0;
   int num_sms = 148;
@@ -1280,6 +1321,12 @@ static void drop_plans(film_handle* h) {
 }
 
 static Plan* get_plan(film_handle* h, int hh, int ww, int align) {
+  {
+    // checked before the cache lookup: a plan built while "any_size" was on must not serve a call made after it is off
+    int H, W, oy, ox;
+    padded_size(hh, ww, align, H, W, oy, ox);
+    check_supported_size(H, W, h->any_size != 0);
+  }
   char key[96];
   snprintf(key, sizeof(key), "%dx%d_a%d_i%d_v%d_l%d_p%d_h%d_m%x_d%d", hh, ww, align > 0 ? align : 0, h->conv_impl, h->conv3x3_v2,
            h->use_lanes, h->conv3x3_2cta, h->conv3x3_halo, h->onepass_mask, h->keep_debug * 256 + h->fuse_flow_head * 64 + h->arena_reuse * 32 + h->mma_straight * 16 + h->plane_skip * 8 + h->conv3x3_dual * 4 +
@@ -1291,7 +1338,7 @@ static Plan* get_plan(film_handle* h, int hh, int ww, int align) {
     p = build_plan(*h->model, hh, ww, align, h->conv_impl, h->keep_debug != 0, h->conv3x3_v2, h->num_sms,
                    h->conv3x3_2cta, h->conv3x3_halo, h->onepass_mask, h->use_lanes != 0, h->fe_conv0_tc | (h->fuse_rgb_head ? 0 : 2) | (h->conv3x3_dual ? 4 : 0) | (h->plane_skip ? 0 : 8) |
                        (h->mma_straight ? 0 : 16) | (h->arena_reuse ? 0 : 32) | (h->fuse_flow_head ? 0 : 64) |
-                       (h->fuse_flow_head >= 2 ? 128 : 0));
+                       (h->fuse_flow_head >= 2 ? 128 : 0), h->any_size != 0);
   } catch (const Error& e0) {
     if (e0.code != FILM_ERR_CUDA) throw;  // only an allocation failure is worth a retry
     // Every cached shape keeps its activation arena (GBs at 1080p).  If a new shape does not fit next to
@@ -1301,7 +1348,7 @@ static Plan* get_plan(film_handle* h, int hh, int ww, int align) {
     p = build_plan(*h->model, hh, ww, align, h->conv_impl, h->keep_debug != 0, h->conv3x3_v2, h->num_sms,
                    h->conv3x3_2cta, h->conv3x3_halo, h->onepass_mask, h->use_lanes != 0, h->fe_conv0_tc | (h->fuse_rgb_head ? 0 : 2) | (h->conv3x3_dual ? 4 : 0) | (h->plane_skip ? 0 : 8) |
                        (h->mma_straight ? 0 : 16) | (h->arena_reuse ? 0 : 32) | (h->fuse_flow_head ? 0 : 64) |
-                       (h->fuse_flow_head >= 2 ? 128 : 0));
+                       (h->fuse_flow_head >= 2 ? 128 : 0), h->any_size != 0);
   }
   if (h->use_graph) {
     cudaGraph_t g = nullptr;
@@ -1463,6 +1510,7 @@ int film_set_option(film_handle* h, const char* name, int value) {
   else if (n == "fuse_flow_head") h->fuse_flow_head = value < 0 ? 0 : (value > 2 ? 2 : value);
   else if (n == "mma_straight") h->mma_straight = value ? 1 : 0;
   else if (n == "arena_reuse") h->arena_reuse = value ? 1 : 0;
+  else if (n == "any_size") h->any_size = value ? 1 : 0;
   else if (n == "clear_plans") drop_plans(h);
   else {
     h->err = "unknown option " + n;
@@ -1493,6 +1541,7 @@ int film_get_option(film_handle* h, const char* name, int* value) {
   else if (!strcmp(name, "conv3x3_halo")) *value = h->conv3x3_halo;
   else if (!strcmp(name, "conv3x3_2cta")) *value = h->conv3x3_2cta;
   else if (!strcmp(name, "keep_debug")) *value = h->keep_debug;
+  else if (!strcmp(name, "any_size")) *value = h->any_size;
   else return FILM_ERR_ARG;
   return FILM_OK;
 }

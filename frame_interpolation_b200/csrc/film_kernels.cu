@@ -393,6 +393,44 @@ cudaError_t launch_act_pool(const sp_t* in_hi, const sp_t* in_lo, int in_C, int 
 }
 
 // ------------------------------------------------------------------------------------------
+// fusion.py:133  tf.image.resize(NEAREST_NEIGHBOR) of a split tensor to a fine grid that is not twice
+// the coarse one.  TF2 index rule in fp32: src = min(floor((dst + 0.5) * (in / out)), in - 1); the
+// scales are fp32 quotients computed by the caller.  One thread copies 8 channels of one pixel.
+// ------------------------------------------------------------------------------------------
+template <bool kHiOnly>
+__global__ void __launch_bounds__(256) k_resize_nearest(const sp_t* __restrict__ in_hi, const sp_t* __restrict__ in_lo,
+                                                        int Hc, int Wc, int C, sp_t* __restrict__ out_hi,
+                                                        sp_t* __restrict__ out_lo, int Hf, int Wf, int64_t n,
+                                                        float sy, float sx) {
+  const int G = C >> 3;
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int g = (int)(i % G);
+  const int64_t p = i / G;
+  const int x = (int)(p % Wf);
+  const int64_t q = p / Wf;
+  const int y = (int)(q % Hf);
+  const int b = (int)(q / Hf);
+  const int ys = min((int)floorf(((float)y + 0.5f) * sy), Hc - 1);
+  const int xs = min((int)floorf(((float)x + 0.5f) * sx), Wc - 1);
+  const int64_t src = (((int64_t)b * Hc + ys) * Wc + xs) * C + g * 8;
+  const int64_t dst = p * C + g * 8;
+  *reinterpret_cast<uint4*>(out_hi + dst) = ldg16(in_hi + src);
+  if (!kHiOnly) *reinterpret_cast<uint4*>(out_lo + dst) = ldg16(in_lo + src);
+}
+
+cudaError_t launch_resize_nearest(const sp_t* in_hi, const sp_t* in_lo, int B, int Hc, int Wc, int C, sp_t* out_hi,
+                                  sp_t* out_lo, int Hf, int Wf, bool hi_only, cudaStream_t st) {
+  if (C % 8) return cudaErrorInvalidValue;
+  const int64_t n = (int64_t)B * Hf * Wf * (C / 8);
+  if (n == 0) return cudaSuccess;
+  const float sy = (float)Hc / (float)Hf, sx = (float)Wc / (float)Wf;
+  if (hi_only) k_resize_nearest<true><<<cdiv(n, 256), 256, 0, st>>>(in_hi, in_lo, Hc, Wc, C, out_hi, out_lo, Hf, Wf, n, sy, sx);
+  else k_resize_nearest<false><<<cdiv(n, 256), 256, 0, st>>>(in_hi, in_lo, Hc, Wc, C, out_hi, out_lo, Hf, Wf, n, sy, sx);
+  return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------
 // Shared gather helpers.
 // TF2 bilinear resize (half-pixel centres):  src = (dst + 0.5) * in/out - 0.5
 // TFA dense_image_warp / interpolate_bilinear border rule: floor clamped to [0, size-2],

@@ -17,8 +17,9 @@ cudaError_t launch_conv0_c3(const float* img, int B, int H, int W, const float* 
 
 // Product path of cfeat_conv_0: register-tiled fp32 direct conv (K = 27 is too short for the tensor cores), reads the
 // fp32 image level, writes the 64-channel split output [B][H][W][64] (hi plane only when `lo_skip`).
-// `pool_out` (nullable): [B][H/2][W/2][3] fp32 -- the 2x2/2 average pool of `img` (util.py:38-44), i.e. the next image
-// pyramid level, written from the input patch the conv has staged anyway (H, W even).
+// `pool_out` (nullable): [B][H/2][W/2][3] fp32 -- the 2x2/2 VALID average pool of `img` (util.py:38-44), i.e. the next
+// image pyramid level, written from the input patch the conv has staged anyway (sizes floor: an odd last row / column
+// is dropped).
 cudaError_t launch_fe_conv0(const float* img, int B, int H, int W, const float* w, const float* bias, sp_t* out_hi,
                             sp_t* out_lo, bool lo_skip, float* pool_out, cudaStream_t st);
 
@@ -33,6 +34,12 @@ cudaError_t launch_image_to_split32(const float* img, int B, int H, int W, sp_t*
 cudaError_t launch_act_pool(const sp_t* in_hi, const sp_t* in_lo, int in_C, int in_c_off, int B,
                             int H, int W, int Cn, sp_t* out_hi, sp_t* out_lo, int out_C,
                             cudaStream_t st);
+
+// fusion.py:133 -- nearest-neighbour resize (TF2 rule, fp32 index arithmetic) of a split tensor
+// [B][Hc][Wc][C] -> [B][Hf][Wf][C], C a multiple of 8: the decoder's up-sampling at levels where the fine grid is
+// not twice the coarse one.  hi_only: only the hi plane is copied (single-pass consumer).
+cudaError_t launch_resize_nearest(const sp_t* in_hi, const sp_t* in_lo, int B, int Hc, int Wc, int C, sp_t* out_hi,
+                                  sp_t* out_lo, int Hf, int Wf, bool hi_only, cudaStream_t st);
 
 // pyramid_flow_estimator.py:154-157 fused: v_up = resize_bilinear(2*v_prev -> HxW);
 // warped[d] = warp(feat[1-d], v_up[d]).  feat/warped are [2][H][W][C] split tensors.

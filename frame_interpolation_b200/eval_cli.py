@@ -1,7 +1,7 @@
 """Benchmark evaluator on the B200 engine -- TF-free counterpart of the reference's `eval/eval_cli.py:88-178`.
 
     python -m frame_interpolation_b200.eval_cli --triplets <dir> --model_path <weights.filmw> \
-        --output_dir <out> [--max_examples N] [--metrics l1,l2,ssim,psnr] [--output_frames]
+        --output_dir <out> [--max_examples N] [--metrics l1,l2,ssim,psnr] [--output_frames] [--align 0 --any_size]
 
 The reference iterates a TFRecord of (x0, y, x1) triplets built by `datasets/create_*_tfrecord.py` from
 folders of three frames (Vimeo-90K `im1/im2/im3.png`, Middlebury `frame10/frame10i11/frame11.png`, ...);
@@ -83,9 +83,13 @@ def main(argv=None) -> int:
     ap.add_argument("--output_frames", action="store_true")
     ap.add_argument("--align", type=int, default=64)
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--any_size", action="store_true",
+                    help="Accept padded frame sizes that are not multiples of 64 (engine option any_size). Use with --align 0 to run frames at their own size, like the reference with align=None.")
     a = ap.parse_args(argv)
     from .interpolator import Interpolator
     interp = Interpolator(a.model_path, align=a.align, device=a.device)
+    if a.any_size:
+        interp.set_option("any_size", 1)
     trip = find_triplets(a.triplets)
     if not trip:
         print(f"[film_b200] no triplet folders under {a.triplets}", file=sys.stderr)

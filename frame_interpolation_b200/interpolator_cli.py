@@ -1,7 +1,7 @@
 """Command line front end with the reference's flags (eval/interpolator_cli.py:85-121) on the B200 engine.
 
     python -m frame_interpolation_b200.interpolator_cli --pattern "photos" --model_path synthetic \
-        --times_to_interpolate 3 [--align 64] [--block_height 2 --block_width 2] [--output_video --fps 30]
+        --times_to_interpolate 3 [--align 64 | --align 0 --any_size] [--block_height 2 --block_width 2] [--output_video --fps 30]
 
 For every directory matching --pattern: the *.png/*.jpg/*.jpeg frames (natural order) are
 interpolated recursively and written to <dir>/interpolated_frames/frame_%03d.png
@@ -38,6 +38,8 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--block_height", type=int, default=1)
     p.add_argument("--block_width", type=int, default=1)
     p.add_argument("--output_video", action="store_true")
+    p.add_argument("--any_size", action="store_true",
+                   help="Accept padded frame sizes that are not multiples of 64 (engine option any_size). Use with --align 0 to run frames at their own size, like the reference with align=None.")
     p.add_argument("--device", type=int, default=None, help="CUDA device ordinal (default: LOCAL_RANK or 0)")
     return p
 
@@ -105,6 +107,8 @@ def main(argv=None) -> int:
     directories = sorted(d for d in glob.glob(args.pattern) if os.path.isdir(d))
     mine = directories[rank::world]            # directories are independent: shard them over ranks
     interpolator = Interpolator(args.model_path, args.align, [args.block_height, args.block_width], device=device)
+    if args.any_size:
+        interpolator.set_option("any_size", 1)
     for d in mine:
         n = process_directory(d, interpolator, args.times_to_interpolate, args.fps, args.output_video)
         print(f"[film_b200] {d}: wrote {n} frames to {d}/interpolated_frames", flush=True)

@@ -85,7 +85,8 @@ FILM_API int film_create(film_handle** out, const char* weights_path, int device
 FILM_API void film_destroy(film_handle* h);
 
 /* Host pointers. x0/x1/out: B*H*W*3 floats. align <= 0 disables padding
- * (eval/interpolator.py:149: `align or None`); then H and W must be multiples of 64.
+ * (eval/interpolator.py:149: `align or None`). A padded size that is not a multiple of 64 needs
+ * option "any_size" (status 4 otherwise); at least 64 rows and columns (status 1 otherwise).
  * Blocks until `out` is written. */
 FILM_API int film_interpolate(film_handle* h, const float* x0, const float* x1, const float* dt,
                      int B, int H, int W, int align, float* out);
@@ -169,12 +170,18 @@ FILM_API int film_profile(film_handle* h, film_profile_t* out);
  *                   after draining the handle's stream.  Plans are cached per shape and never evicted
  *                   otherwise, except that a shape whose arena cannot be allocated triggers one
  *                   drop-and-retry before FILM_ERR_CUDA is returned. */
-/*   "onepass_mask": precision plan -- bit s selects the single-pass product (A_hi x W_hi, fp16 operands, fp32
+/*   "any_size"    : 1 = padded frame sizes that are not multiples of 64 are computed like the reference graph does
+ *                   (VALID pooling floors; flows and the decoder resize to each level's size), from 64 rows / columns
+ *                   up; 0 (default) = they are refused with status 4.  Checked on every call, before the plan cache:
+ *                   turning it off refuses such a size again even when its plan is cached.  It never changes how a
+ *                   64-aligned size is computed.
+ *   "onepass_mask": precision plan -- bit s selects the single-pass product (A_hi x W_hi, fp16 operands, fp32
  *                   accumulate) for stage s (film_stage_count / film_stage_name); every other conv runs the
  *                   three-pass split product.  The default is the measured plan of DESIGN.md section 3;
  *                   0 = every conv three-pass (fp32-grade).  "onepass_default" (any value) restores it. */
 FILM_API int film_set_option(film_handle* h, const char* name, int value);
-/* Reads back an integer option ("onepass_mask", "onepass_default", "conv3x3_halo", "conv3x3_2cta", "keep_debug"). */
+/* Reads back an integer option ("onepass_mask", "onepass_default", "conv3x3_halo", "conv3x3_2cta", "keep_debug",
+ * "any_size"). */
 FILM_API int film_get_option(film_handle* h, const char* name, int* value);
 
 /* Stages of the precision plan: film_stage_count() names ("fe_i0_k01", "flow_L3", "fus2_c1", ...), index =
